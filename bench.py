@@ -2,6 +2,7 @@
 """bench.py - benchmarks of the ELD synthetic-noise training path on B200 (one process per GPU).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload train|infer|noise|fullframe] [--impl reference]
+                    [--dump-outputs DIR]
 
 Workloads = BASELINE.json configs (a "frame" is one 4x512x512 packed raw tensor unless stated):
     train      configs[2]  G+P* noise -> U-Net fwd + L1 + bwd -> (all-reduce) -> Adam, batch 8 per GPU, bf16   [default]
@@ -10,7 +11,8 @@ Workloads = BASELINE.json configs (a "frame" is one 4x512x512 packed raw tensor 
     fullframe  configs[4]  4-camera sweep over 4256 x 2848 full frames (packed 4 x 1424 x 2128), noise synthesis only
 Prints ONE JSON line on rank 0.  DESIGN.md section 7 defines value / e2e / roofline / roofline_noise / onbox_baseline /
 cpu_baseline.  `--impl reference` times the reference's own CPU path (numpy / torch-CPU port under oracle/) and never
-imports the product package.
+imports the product package.  `--dump-outputs DIR` saves what the last timed step computed as DIR/<name>.npy (rank 0);
+the inputs depend only on the arguments, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -27,6 +29,8 @@ SONY = (2.2881136684755243, 6.4508722699636545, 15583, 208.9766365993794)
 FRAME_PX = 4 * 512 * 512
 FULL_H, FULL_W = 1424, 2128                      # packed full frame of a 2848 x 4256 sensor (config 5)
 METRIC = 'raw frames/sec (noise+U-Net)'
+DUMP_SAMPLE = 1 << 22                            # elements kept of a larger output: 16 MB in f32, <= 4 outputs per workload
+DUMP_LIMIT = 64 << 20
 
 
 def peaks():
@@ -233,24 +237,45 @@ def reference_arm(a):
         fps = noise_fps
         sample = '%d frames/step of 4x%dx%d in a %d-process pool, numpy port of noise.py model %s' % (per_step, h, wd, per_step, model)
     elif w == 'infer':
-        fps, nthr = cpu_infer_fps(steps=max(1, min(a.steps, 5)))
-        sample = 'reference module torch CPU fp32 forward 1x4x512x512 on %d threads (best of 16/32/64; nproc = %d)' % (nthr, nproc)
+        fps, nthr = cpu_infer_fps(steps=a.steps)
+        sample = ('reference module torch CPU fp32 forward 1x4x512x512 x %d steps on %d threads (best of 16/32/64; nproc = %d)'
+                  % (a.steps, nthr, nproc))
     else:
         from oracle import unet_ref
-        k = max(1, min(a.steps, 3))
-        fps_unet, nthr = unet_ref.cpu_train_fps_best(steps=k, warmup=1, batch=1)
+        fps_unet, nthr = unet_ref.cpu_train_fps_best(steps=a.steps, warmup=1, batch=1)
         fps = 1.0 / (1.0 / noise_fps + 1.0 / fps_unet)
         sample = ('noise: %d frames/step in a %d-process pool (%.1f frames/s); U-Net: torch CPU fp32 fwd+L1+bwd+Adam batch 1 x %d '
                   'steps on %d threads (%.2f frames/s; best of min(nproc, 16/32/64); nproc = %d); legs summed serially'
-                  % (per_step, nproc, noise_fps, k, nthr, fps_unet, nproc))
+                  % (per_step, nproc, noise_fps, a.steps, nthr, fps_unet, nproc))
     out.update({'value': fps, 'ms_per_step': 1000.0 * a.batch / fps,
                 'cpu_baseline': {'value': fps, 'unit': 'frames/s', 'cores': nproc, 'kind': 'port', 'sample': sample},
-                'e2e': {'value': fps, 'unit': 'frames/s', 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0},
+                'e2e': {'value': fps, 'unit': 'frames/s', 'steps': a.steps, 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0},
                 'gpu_launches': 0})
     print(json.dumps(out))
 
 
 # ------------------------------------------------------------------------------------------------
+def dump_outputs(d, outs):
+    """outs: {name: tensor} of one step -> d/<name>.npy, float32 (float64 kept), in the output's shape.  An output of
+    n > DUMP_SAMPLE elements is saved flat as exactly DUMP_SAMPLE of its elements: element j is the flat element
+    j * n // DUMP_SAMPLE + floor(u_j * size of that range), u = RandomState(0).random_sample(DUMP_SAMPLE), so the sample
+    spreads evenly over the output and depends only on n."""
+    import numpy as np
+    import torch
+    os.makedirs(d, exist_ok=True)
+    total = 0
+    for name, t in sorted(outs.items()):
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            edges = np.arange(DUMP_SAMPLE + 1) * t.numel() // DUMP_SAMPLE
+            idx = edges[:-1] + (np.random.RandomState(0).random_sample(DUMP_SAMPLE) * np.diff(edges)).astype(np.int64)
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        arr = t.cpu().numpy().astype(np.float64 if t.dtype == torch.float64 else np.float32)
+        total += arr.nbytes
+        assert total <= DUMP_LIMIT, 'outputs exceed %d bytes' % DUMP_LIMIT
+        np.save(os.path.join(d, name + '.npy'), arr)
+
+
 def make_noise_steps(a, dev, rank, world, full):
     import numpy as np
     import torch
@@ -276,7 +301,7 @@ def make_noise_steps(a, dev, rank, world, full):
     dev_out = torch.empty_like(dev_in)
 
     def step(i):
-        nm.batch_gpu(clean[i & 1], params=plist, frame_id0=(i * world + rank) * B, out=noisy[i & 1])
+        return {'noisy': nm.batch_gpu(clean[i & 1], params=plist, frame_id0=(i * world + rank) * B, out=noisy[i & 1])}
 
     def step_e2e(i):
         dev_in.copy_(host_in, non_blocking=True)
@@ -299,12 +324,17 @@ def main():
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-onbox', action='store_true', help='skip the torch-eager/cuDNN on-box baseline')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write what the last timed step computed as DIR/<name>.npy')
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
     if a.batch is None:
         a.batch = {'train': 8, 'infer': 1, 'noise': 32, 'fullframe': 4}[a.workload]
     a.warmup = max(a.warmup, 3)
 
     if a.impl == 'reference':
+        if a.dump_outputs:
+            ap.error('--dump-outputs saves the product path; --impl reference has none')
         return reference_arm(a)
 
     import torch
@@ -352,8 +382,9 @@ def main():
     if sampler is not None:
         sampler.window(True)
     ev[0].record()
-    for i in range(a.steps):
+    for i in range(a.steps - 1):
         step(a.warmup + i)
+    last = step(a.warmup + a.steps - 1)             # only the last step's outputs outlive it, for --dump-outputs
     ev[1].record()
     import ctypes
     probe = torch.zeros(1, device=dev)
@@ -369,6 +400,8 @@ def main():
         clocks['sm_mhz_device_probe'] = float(probe.item())
     ms = ev[0].elapsed_time(ev[1])
     launches = _lib.launch_count(local) - l0
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, last)              # before the end-to-end steps below move the weights on
     t = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -409,7 +442,7 @@ def main():
            'steps': a.steps, 'warmup': a.warmup, 'ms_per_step': ms / a.steps, 'higher_is_better': True,
            'scaling': 'weak', 'vs_baseline': None, 'dtype': dtype, 'data': 'synthetic',
            'config': config_dict(a), 'clocks': clocks,
-           'e2e': {'value': e2e_value, 'unit': 'frames/s', 'h2d_bytes_per_step': h2d, 'd2h_bytes_per_step': d2h},
+           'e2e': {'value': e2e_value, 'unit': 'frames/s', 'steps': e2e_steps, 'h2d_bytes_per_step': h2d, 'd2h_bytes_per_step': d2h},
            'gpu_launches': launches, 'roofline': roof}
     if a.workload == 'fullframe':
         out['equiv_512_frames_per_s'] = value * FULL_H * FULL_W / (512.0 * 512.0)

@@ -12,7 +12,8 @@ pytestmark = pytest.mark.gpu
 @pytest.fixture(scope='module')
 def torch():
     import torch as t
-    assert t.cuda.is_available()
+    if not t.cuda.is_available():
+        pytest.skip('no GPU')
     return t
 
 
