@@ -45,6 +45,7 @@ def _declare(lib):
     lib.eld_noise_packed_aug.argtypes = [vp, vp, vp, vp, i32, i32, i32, c.POINTER(NoiseParams), u32, u64, u64, i32,
                                          c.POINTER(c.c_uint8), vp]
     lib.eld_eval_correct_psnr.argtypes = [vp, vp, vp, vp, i32, c.c_size_t, i32, vp, vp, vp, vp]
+    lib.eld_eval_ssim.argtypes = [vp, vp, vp, i32, i32, i32, i32, vp, vp, vp]
     from . import _unet_abi
     _unet_abi.declare(lib)
 

@@ -294,14 +294,32 @@ class ELDModel(BaseModel):
             ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)), 'eld_eval_correct_psnr')
         return out, psnr, gain
 
+    def eval_ssim(self, predict, target):
+        """tensor2im (ELD_model.py:23-38) + skimage's structural_similarity(data_range=255, multichannel=True) with its
+        defaults (util/index.py:80) per frame of NCHW fp32 tensors, on the device (csrc/eval.cu, two launches, no host
+        synchronisation).  A 1-frame target is broadcast over the batch like eval_metrics.  Returns ssim[n] (f32)."""
+        import ctypes
+        from . import _lib
+        predict, target = predict.contiguous(), target.contiguous()
+        n, c, h, w = predict.shape
+        if target.shape[0] == 1 and n != 1:
+            target = target.expand_as(predict).contiguous()
+        scratch = torch.empty(n * c, dtype=torch.float64, device=predict.device)
+        ssim = torch.empty(n, dtype=torch.float32, device=predict.device)
+        _lib.check(_lib.load().eld_eval_ssim(
+            _lib.ctx(predict.device.index or 0), predict.data_ptr(), target.data_ptr(), n, c, h, w, scratch.data_ptr(),
+            ssim.data_ptr(), ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)), 'eld_eval_ssim')
+        return ssim
+
     def illuminance_correct(self, predict, source):
         return self.eval_metrics(predict, source, correct=True)[0]
 
     def eval(self, data, savedir=None, suffix=None, correct=False, crop=True, frame_id=None, **kwargs):
         """ELDModelBase.eval (ELD_model.py:203-243) without the rawpy / PIL visualisation: centre 512x512 crop
-        (util.crop_center), forward (or forward_chop), optional illuminance correction, PSNR of the output and of the
-        input against the target exactly as tensor2im + quality_assess compute them - all on the device (csrc/eval.cu);
-        one host read of the final scalars.  Only the 1st frame is assessed, like the reference (tensor2im takes [0])."""
+        (util.crop_center), forward (or forward_chop), optional illuminance correction, PSNR and SSIM of the output and
+        of the input against the target exactly as tensor2im + quality_assess compute them - all on the device
+        (csrc/eval.cu); one host read of the final scalars.  Only the 1st frame is assessed, like the reference
+        (tensor2im takes [0])."""
         self._eval()
         self.set_input(data, 'eval')
         with torch.no_grad():
@@ -313,9 +331,11 @@ class ELDModel(BaseModel):
             out = self.forward_chop(x) if self.opt.chop else self._padded_forward(x)
             out, psnr, _ = self.eval_metrics(out.contiguous(), t, correct=correct)
             _, psnr_in, _ = self.eval_metrics(x, t, correct=False)
+            ssim = self.eval_ssim(out[:1], t[:1])
+            ssim_in = self.eval_ssim(x[:1], t[:1])
             self.output = out
-            both = torch.stack([psnr[0], psnr_in[0]]).cpu()
-        return {'PSNR': float(both[0]), 'PSNR_input': float(both[1])}
+            r = torch.stack([psnr[0], psnr_in[0], ssim[0], ssim_in[0]]).cpu()
+        return {'PSNR': float(r[0]), 'PSNR_input': float(r[1]), 'SSIM': float(r[2]), 'SSIM_input': float(r[3])}
 
     def test(self, data, savedir=None, **kwargs):
         self._eval()

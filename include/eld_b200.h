@@ -142,6 +142,19 @@ int eld_isp_process(eld_ctx* ctx, const float* packed, float* rgb, int n, int h,
 int eld_eval_correct_psnr(eld_ctx* ctx, const float* pred, const float* target, float* out, int n, size_t per_frame,
                           int correct, double* scratch, float* psnr, float* gain, void* stream);
 
+/* SSIM of ELDModelBase.eval: tensor2im (:23-38) + skimage's structural_similarity(data_range = 255,
+ * multichannel = True) with its defaults (util/index.py:80), per frame f of x and y, device f32 [n][c][h][w]:
+ *   per plane, on a = clip(255 x,0,255), b = clip(255 y,0,255) (no rounding): 7x7 box means ux, uy, uxx, uyy, uxy;
+ *   vx = 49/48 (uxx - ux^2), vy = 49/48 (uyy - uy^2), vxy = 49/48 (uxy - ux uy); C1 = (0.01*255)^2, C2 = (0.03*255)^2;
+ *   S = (2 ux uy + C1)(2 vxy + C2) / ((ux^2 + uy^2 + C1)(vx + vy + C2)), averaged over the (h-6)(w-6) positions whose
+ *   window lies inside the plane (skimage's crop by 3: its reflected border never enters the result);
+ *   ssim[f] = mean over the c channels.  Symmetric in x, y up to fp32 rounding.  Window sums in fp32 (of the values
+ *   less 127.5), sums over positions in double.
+ * h, w >= 7 (skimage's 7x7 window), n, c >= 1; x, y contiguous, with no alignment requirement on them or on w.
+ * scratch: device, n * c doubles (zeroed here).  ssim: device f32 [n].  Two launches, no host synchronisation. */
+int eld_eval_ssim(eld_ctx* ctx, const float* x, const float* y, int n, int c, int h, int w, double* scratch,
+                  float* ssim, void* stream);
+
 /* Number of kernels the library has launched through this ctx since creation (bench.py's
  * gpu_launches evidence). */
 int64_t eld_launch_count(const eld_ctx* ctx);
